@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — step ready-evaluations/sec of the StoryRun DAG frontier pass.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--config 3]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--config 3] [--dump-outputs DIR]
 
 A "step" is one frontier pass over one batch of synthetic StoryRuns: BASELINE.json
 configs[2] — 100k StoryRuns x 256 steps, random DAG with in-degree 4 — per GPU (weak
@@ -52,7 +52,7 @@ F_COND, F_DECISION, F_CHILD = 0x1, 0x2, 0x4
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=60)
+    ap.add_argument("--steps", type=int, default=60, help="frontier passes in each timed repetition (see --reps)")
     ap.add_argument("--warmup", type=int, default=6)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", type=int, default=3, help="BASELINE.json config index (2..5), default 3 = configs[2]")
@@ -68,7 +68,13 @@ def parse():
     ap.add_argument("--ncu", action="store_true", help="profiling run: few eager passes, no e2e / cpu / extra legs")
     ap.add_argument("--no-graph", action="store_true", help="launch every pass eagerly instead of replaying a CUDA graph")
     ap.add_argument("--unroll", type=int, default=0, help="passes captured per CUDA graph (default: the largest divisor of --steps <= 64)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed pass returned (result records, counts, expansion "
+                         "tuples) as DIR/<name>.npy in float32 / float64 (rank 0's shard on several GPUs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 CFG_N = {2: 10_000, 3: 100_000, 4: 100_000, 5: 125_000}
@@ -276,13 +282,38 @@ def set_sequence(U, ROT):
     return seq
 
 
+DUMP_BYTES = 60_000_000   # data of all --dump-outputs files together (with the .npy headers: under 64 MB)
+
+
+def dump_outputs(out_dir, arrays, budget=DUMP_BYTES):
+    """Writes each array of `arrays` (name -> integer array, rows first) as out_dir/<name>.npy: float32 for 8- and 16-bit
+    values, float64 for wider ones, so every value is exact.  The smallest arrays go first and each array may use an equal
+    share of what the earlier ones left of `budget`; one that does not fit is replaced by a sample of its rows drawn with a
+    fixed seed, and the sampled row numbers are written beside it as <name>_rows.npy (float64)."""
+    os.makedirs(out_dir, exist_ok=True)
+    conv = {k: (np.ascontiguousarray(a), np.float32 if a.dtype.itemsize <= 2 else np.float64) for k, a in arrays.items()}
+    left = budget
+    for i, name in enumerate(sorted(conv, key=lambda k: conv[k][0].size * np.dtype(conv[k][1]).itemsize)):
+        a, ft = conv[name]
+        share = left // (len(conv) - i)
+        row_bytes = (a.size // max(a.shape[0], 1)) * np.dtype(ft).itemsize
+        if a.size * np.dtype(ft).itemsize > share:
+            k = share // (row_bytes + 8)
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], size=k, replace=False))
+            np.save(os.path.join(out_dir, name + "_rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+            left -= 8 * k
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(ft))
+        left -= a.size * np.dtype(ft).itemsize
+
+
 def run_config(g, cfg, n_runs, ROT, steps, warmup, reps, headline):
     """Builds the inputs of one configuration on this rank, checks the full batch against the oracle, times it.
     Returns (summary dict, live objects for the headline's extra legs)."""
     import torch
     import torch.distributed as dist
     from bobrapet_b200 import _abi as A, Frontier, synth
-    from bobrapet_b200.records import make_layout
+    from bobrapet_b200.records import EXP_DTYPE, make_layout
     from bobrapet_b200.sharding import CountExchange, global_offsets
     args, dev, world, rank = g.args, g.dev, g.world, g.rank
     S = CFG_S[cfg]
@@ -432,6 +463,14 @@ def run_config(g, cfg, n_runs, ROT, steps, warmup, reps, headline):
         return t.cpu().numpy()
 
     reg = timed(graph, True, reps)
+    last = seq[-1] if graph is not None else (steps - 1) % ROT   # the input set of the last timed pass
+    outputs = None
+    if headline and args.dump_outputs and rank == 0:
+        _, _, d_result, d_counts, _, d_exp, exp_cap = sets[last]
+        outputs = {"result": d_result.cpu().numpy(), "counts": d_counts.cpu().numpy()}
+        if exp_cap:
+            e = d_exp.cpu().numpy().view(EXP_DTYPE).reshape(-1)[:min(int(outputs["counts"][2]), exp_cap)]
+            outputs["expansion"] = np.stack([e["run"], e["step"], e["branch"]], axis=1).astype(np.uint32)
     ms = float(np.median(reg))
     exposed_us = None
     if graph_nc is not None:
@@ -446,8 +485,8 @@ def run_config(g, cfg, n_runs, ROT, steps, warmup, reps, headline):
             del graph_plain
         except Exception as e:
             sys.stderr.write("bench: plain-pass graph failed (%s)\n" % e)
-    counts_host = sets[seq[-1] if graph is not None else (steps - 1) % ROT][3].cpu().numpy().tolist()
-    offsets = global_offsets(gathered[seq[-1] if graph is not None else (steps - 1) % ROT], rank) if world > 1 else None
+    counts_host = sets[last][3].cpu().numpy().tolist()
+    offsets = global_offsets(gathered[last], rank) if world > 1 else None
 
     # ---- kernel-only duration: event pair around single launches (carries the launch gaps: reported, not used for frac)
     stream = torch.cuda.current_stream()
@@ -522,6 +561,7 @@ def run_config(g, cfg, n_runs, ROT, steps, warmup, reps, headline):
     live.fr, live.sets, live.L, live.graph, live.graph_nc = fr, sets, L, graph, graph_nc
     live.timed_launches = int(round(steps * launches_per_pass))
     live.topology_put_ms, live.counts0 = put_ms, counts_host
+    live.outputs = outputs
     return out, live
 
 
@@ -701,7 +741,7 @@ def main():
     e2e = None
     if not args.no_e2e:
         e2e = e2e_legs(g, live, n_runs, S, args.steps)
-    timed_launches = live.timed_launches
+    timed_launches, outputs = live.timed_launches, live.outputs
     release(live)
 
     # ---- the other configurations BASELINE.json names: cfg4 at every N, cfg5 (125k runs x 1024 steps per GPU = 1M x 1024 at 8)
@@ -751,6 +791,8 @@ def main():
 
     rc = 0
     if rank == 0:
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         line = {
             "metric": METRIC, "value": head["value"], "unit": UNIT, "n_gpus": n_gpus, "steps": args.steps, "warmup": args.warmup,
             "ms_per_step": head["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,

@@ -2,8 +2,11 @@
 all-gather of the per-shard counts per pass, and limiters whose totals are all-reduced across the shards.
 
 On a 1-GPU box the group has one shard (the communicator has one rank); with 2+ GPUs every G up to the device count runs."""
+import functools
+
 import numpy as np
 import pytest
+import torch  # before any group exists: bf_group_create dlopens libnccl.so.2, and torch must load its own build of it first
 
 from bobrapet_b200 import _abi as A
 from bobrapet_b200 import FrontierGroup, synth
@@ -16,13 +19,9 @@ from tests.test_gpu_limiters import _running_and_demand
 pytestmark = pytest.mark.gpu
 
 
-def _device_counts():
-    import torch
-    n = torch.cuda.device_count()
-    return [g for g in (1, 2, 3, 4, 8) if g <= n]
-
-
-@pytest.fixture(params=_device_counts())
+# Group sizes are fixed here rather than read from the box, so that a test has the same ids on every machine: the one-device
+# variants run wherever there is a GPU, and test_groups_of_several_devices runs the same checks on 2, 3, 4 and 8 devices.
+@pytest.fixture(params=[1])
 def group(request):
     g = FrontierGroup(list(range(request.param)))
     yield g
@@ -108,6 +107,22 @@ def test_group_rejects_bad_arguments(group):
     dup = (C.c_int32 * 2)(0, 0)
     assert lib.bf_group_create(C.byref(g), dup, 2, None) == A.BF_EINVAL          # the same device twice
     assert lib.bf_group_create(C.byref(g), dup, 0, None) == A.BF_EINVAL
+
+
+def test_groups_of_several_devices():
+    """the group tests above on every group of 2, 3, 4 and 8 devices the box holds, a fresh group for each check"""
+    sizes = [n for n in (2, 3, 4, 8) if n <= torch.cuda.device_count()]
+    if not sizes:
+        pytest.skip("needs at least 2 GPUs")
+    checks = [test_group_eval_sharded_topologies, test_group_rejects_bad_arguments] + \
+             [functools.partial(test_group_schedule_holds_limits_across_shards, seed=s) for s in range(3)]
+    for n in sizes:
+        for check in checks:
+            g = FrontierGroup(list(range(n)))
+            try:
+                check(g)
+            finally:
+                g.close()
 
 
 def test_queue_max_priority_base_blocks_lower_priority_runs():
