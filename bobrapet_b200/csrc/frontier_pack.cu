@@ -62,56 +62,58 @@ struct WalkCtx {
 };
 
 // K items at once (independent load chains); FMT as in kernel_common.cuh — the caller guarantees that every live run
-// of the group has this row format (else it takes walk_items_any).
-// AL (byte-entry rows of four, 8 words per run): the status bytes of a run start on a 256-byte boundary, so the address of a
-// dependency's status byte is ONE byte permute — byte k of the row word over the low byte of the base — instead of an
-// extract and an add.  Fixed-width rows exist for every step of a word, so all 32 lanes fetch and the candidate word (the
-// same in every lane after the shuffle) masks the ballot instead of every lane's predicate.
+// of the group has this row format (else it takes walk_items_any).  Items are taken from the highest lane down (one FLO
+// per item); every item delivers to its own lane, so the order does not matter.
+// Fixed-width rows exist for every step of a word, so all 32 lanes fetch and ballot; the ballots are not masked here — the
+// owner lane masks its two words with its own candidate word once, after the walk (walk_items).  For every byte a fixed-width
+// row can name (a step < S, col_idx is validated at upload, or PAD) the status byte is 0, 1 or 3 (FD is a subset of U below S,
+// and PAD is 0), so the OR of a row's bytes is 0 when every need is met and above 1 when one has failed.
+// AL (byte-entry rows of four, 8 words per run): the owner lane of an item publishes `own` = (its row base << 14) | (its run's
+// status base >> 8) (walk_items); one shuffle gives every lane both.  The status bytes of a run start on a 256-byte boundary,
+// so the address of a dependency's status byte is ONE byte permute: byte k of the row word, then bytes 0 and 1 of `own`
+// (status base bits 8 .. 17; bits 14 and 15 of `own` are row-base bits 0 and 1, zero for a 4-byte aligned row), then the
+// sign of byte 1 (bit 15 = 0) as the zero top byte.
 template <int K, int FMT, bool NEED_FD, bool AL = false>
-DI void walk_items_k(uint32_t lane, uint32_t CAND, uint32_t& todo, uint32_t lg, const WalkCtx& C, uint32_t& met_w, uint32_t& fd_w) {
+DI void walk_items_k(uint32_t lane, uint32_t CAND, uint32_t own, uint32_t& todo, uint32_t lg, const WalkCtx& C, uint32_t& met_w,
+                     uint32_t& fd_w) {
   const uint32_t wmask = (1u << lg) - 1u;
-  uint32_t L[K], p[K], n[K], wv[K], st[K], cw[K], x[K][4];
+  uint32_t L[K], p[K], n[K], wv[K], st[K], x[K][4];
   bool c[K];
 #pragma unroll
   for (int k = 0; k < K; ++k) {
-    L[k] = __ffs(todo) - 1;
-    todo &= todo - 1;
+    L[k] = 31u - __clz(todo);
+    todo &= bmsk_clamp(0u, L[k]);   // clears bit L and above
   }
   if (AL && FMT == FMT_ELL4B) {
 #pragma unroll
     for (int k = 0; k < K; ++k) {
-      cw[k] = __shfl_sync(FULL, CAND, L[k]);
-      const uint32_t g = L[k] >> 3, i = (L[k] & 7u) * 32u + lane;
-      st[k] = C.st0 + g * 256u;
-      p[k] = C.col0 + g * C.topo_buf + i * 4u;
+      st[k] = __shfl_sync(FULL, own, L[k]);
+      n[k] = lds_u32((st[k] >> 14) + lane * 4u);   // the row of step (L & 7) * 32 + lane: four byte entries
     }
 #pragma unroll
-    for (int k = 0; k < K; ++k) n[k] = lds_u32(p[k]);   // the row: four byte entries
-#pragma unroll
     for (int k = 0; k < K; ++k)
-      wv[k] = lds_u8(__byte_perm(n[k], st[k], 0x7650)) | lds_u8(__byte_perm(n[k], st[k], 0x7651)) |
-              lds_u8(__byte_perm(n[k], st[k], 0x7652)) | lds_u8(__byte_perm(n[k], st[k], 0x7653));
+      wv[k] = lds_u8(prmt(n[k], st[k], 0xD540u)) | lds_u8(prmt(n[k], st[k], 0xD541u)) | lds_u8(prmt(n[k], st[k], 0xD542u)) |
+              lds_u8(prmt(n[k], st[k], 0xD543u));
 #pragma unroll
     for (int k = 0; k < K; ++k) {
-      const uint32_t m = __ballot_sync(FULL, (wv[k] & 1u) == 0) & cw[k];
-      if (lane == L[k]) met_w = m;
-      if (NEED_FD) {
-        const uint32_t f = __ballot_sync(FULL, (wv[k] & 2u) != 0) & cw[k];
-        if (lane == L[k]) fd_w = f;
+      const uint32_t m = __ballot_sync(FULL, wv[k] == 0);
+      const uint32_t f = NEED_FD ? __ballot_sync(FULL, wv[k] > 1u) : 0u;
+      if (lane == L[k]) {
+        met_w = m;
+        if (NEED_FD) fd_w = f;
       }
     }
     return;
   }
 #pragma unroll
   for (int k = 0; k < K; ++k) {
-    cw[k] = __shfl_sync(FULL, CAND, L[k]);
     const uint32_t g = L[k] >> lg, i = (L[k] & wmask) * 32u + lane;
-    c[k] = (cw[k] >> lane) & 1u;
     if (fmt_traits<FMT>::fixed) {
       st[k] = C.st0 + g * C.st_stride;
       p[k] = C.col0 + g * C.topo_buf + i * fmt_traits<FMT>::row_bytes;   // rows exist for every step of the word (device_record.h)
       n[k] = (uint32_t)(FMT & 0xFF);
     } else {
+      c[k] = (__shfl_sync(FULL, CAND, L[k]) >> lane) & 1u;
       const uint4 t = lds_v4(C.tab_a + g * 16u);
       st[k] = t.z;
       row_locate<FMT>(c[k], i, t.y, t.x, p[k], n[k]);
@@ -123,12 +125,12 @@ DI void walk_items_k(uint32_t lane, uint32_t CAND, uint32_t& todo, uint32_t lg, 
   for (int k = 0; k < K; ++k) wv[k] = row_status<FMT>(p[k], n[k], x[k], st[k]);
 #pragma unroll
   for (int k = 0; k < K; ++k) {
-    if (fmt_traits<FMT>::fixed) {   // every lane holds a real row: mask the ballot with the (lane-uniform) candidate word
-      const uint32_t m = __ballot_sync(FULL, (wv[k] & 0x01010101u) == 0) & cw[k];
-      if (lane == L[k]) met_w = m;
-      if (NEED_FD) {
-        const uint32_t f = __ballot_sync(FULL, (wv[k] & 0x02020202u) != 0) & cw[k];
-        if (lane == L[k]) fd_w = f;
+    if (fmt_traits<FMT>::fixed) {   // wv = OR of the row's status bytes (0, 1 or 3)
+      const uint32_t m = __ballot_sync(FULL, wv[k] == 0);
+      const uint32_t f = NEED_FD ? __ballot_sync(FULL, wv[k] > 1u) : 0u;
+      if (lane == L[k]) {
+        met_w = m;
+        if (NEED_FD) fd_w = f;
       }
     } else {
       const uint32_t m = __ballot_sync(FULL, c[k] && (wv[k] & 0x01010101u) == 0);
@@ -145,11 +147,18 @@ template <int FMT, bool NEED_FD, bool AL = false>
 DI void walk_items(uint32_t lane, uint32_t CAND, uint32_t lg, const WalkCtx& C, uint32_t& met_w, uint32_t& fd_w) {
   met_w = 0;
   fd_w = 0;
+  uint32_t own = 0;
+  if (AL) {   // Wq = 8: lane = g * 8 + w; shared-window addresses are below 2^18 (at most 227 KB of shared memory per block)
+    const uint32_t g = lane >> 3, w = lane & 7u;
+    own = ((C.col0 + g * C.topo_buf + w * 128u) << 14) | ((C.st0 + g * 256u) >> 8);
+  }
   uint32_t todo = __ballot_sync(FULL, CAND != 0);  // (run, word) pairs with at least one candidate step
-  while (__popc(todo) >= WALK_K) walk_items_k<WALK_K, FMT, NEED_FD, AL>(lane, CAND, todo, lg, C, met_w, fd_w);
+  while (__popc(todo) >= WALK_K) walk_items_k<WALK_K, FMT, NEED_FD, AL>(lane, CAND, own, todo, lg, C, met_w, fd_w);
   if (WALK_K > 2)
-    if (__popc(todo) >= 2) walk_items_k<2, FMT, NEED_FD, AL>(lane, CAND, todo, lg, C, met_w, fd_w);
-  if (todo) walk_items_k<1, FMT, NEED_FD, AL>(lane, CAND, todo, lg, C, met_w, fd_w);
+    if (__popc(todo) >= 2) walk_items_k<2, FMT, NEED_FD, AL>(lane, CAND, own, todo, lg, C, met_w, fd_w);
+  if (todo) walk_items_k<1, FMT, NEED_FD, AL>(lane, CAND, own, todo, lg, C, met_w, fd_w);
+  met_w &= CAND;   // the fixed-width ballots cover all 32 steps of a word
+  fd_w &= CAND;
 }
 
 // mixed row formats inside one group (rare): one item at a time, format read from the item's table entry
@@ -163,13 +172,15 @@ DI void walk_items_any(uint32_t lane, uint32_t CAND, uint32_t lg, const WalkCtx&
     const int fmt = fmt_of(meta >> 16, meta & 0xFFFFu);  // warp-uniform
     uint32_t one = todo & (0u - todo);
     todo ^= one;
-    if (fmt == FMT_ELL4B) walk_items_k<1, FMT_ELL4B, NEED_FD>(lane, CAND, one, lg, C, met_w, fd_w);
-    else if (fmt == FMT_ELL2B) walk_items_k<1, FMT_ELL2B, NEED_FD>(lane, CAND, one, lg, C, met_w, fd_w);
-    else if (fmt == FMT_ELL4) walk_items_k<1, FMT_ELL4, NEED_FD>(lane, CAND, one, lg, C, met_w, fd_w);
-    else if (fmt == FMT_CSR4) walk_items_k<1, FMT_CSR4, NEED_FD>(lane, CAND, one, lg, C, met_w, fd_w);
-    else if (fmt == FMT_ELL2) walk_items_k<1, FMT_ELL2, NEED_FD>(lane, CAND, one, lg, C, met_w, fd_w);
-    else walk_items_k<1, FMT_CSRL, NEED_FD>(lane, CAND, one, lg, C, met_w, fd_w);
+    if (fmt == FMT_ELL4B) walk_items_k<1, FMT_ELL4B, NEED_FD>(lane, CAND, 0u, one, lg, C, met_w, fd_w);
+    else if (fmt == FMT_ELL2B) walk_items_k<1, FMT_ELL2B, NEED_FD>(lane, CAND, 0u, one, lg, C, met_w, fd_w);
+    else if (fmt == FMT_ELL4) walk_items_k<1, FMT_ELL4, NEED_FD>(lane, CAND, 0u, one, lg, C, met_w, fd_w);
+    else if (fmt == FMT_CSR4) walk_items_k<1, FMT_CSR4, NEED_FD>(lane, CAND, 0u, one, lg, C, met_w, fd_w);
+    else if (fmt == FMT_ELL2) walk_items_k<1, FMT_ELL2, NEED_FD>(lane, CAND, 0u, one, lg, C, met_w, fd_w);
+    else walk_items_k<1, FMT_CSRL, NEED_FD>(lane, CAND, 0u, one, lg, C, met_w, fd_w);
   }
+  met_w &= CAND;
+  fd_w &= CAND;
 }
 
 // CD: cond and/or decision codes present   XO: any of fail/needs_cond/skip_dep/phase_out requested
@@ -459,23 +470,27 @@ __global__ void __launch_bounds__(32 * PACK_MAX_WARPS, PACK_MIN_BLOCKS) frontier
     const int my_fmt = fmt_of(ell, max_deg);
     const int fmt0 = __shfl_sync(FULL, live ? my_fmt : -1, __ffs(__ballot_sync(FULL, live) | 0x80000000u) - 1);  // format of the first live run
     const bool mixed = __any_sync(FULL, live && my_fmt != fmt0);
+    const uint32_t my_st = st0_a + g * st_stride;
     __syncwarp();
+    {
+      // every lane writes the 32 bytes of its own word, 16 steps per store; the half a lane stores first follows lane bit 2,
+      // so that at Wq = 8 (words 32 bytes apart) the 8 lanes of each store phase cover all 32 banks
+      const uint32_t hs = lane & 4u ? 16u : 0u;
+      const uint32_t u = __funnelshift_r(U, U, hs), f = __funnelshift_r(FD, FD, hs);   // step hs + j at bit j
 #pragma unroll
-    for (uint32_t it = 0; it < 4; ++it) {
-      const uint32_t item = it * 32 + lane;  // 8 steps: byte (item & 3) of the word held by lane item >> 2
-      const uint32_t sh = (item & 3u) * 8u;
-      const uint32_t ub = __shfl_sync(FULL, U, item >> 2) >> sh;
-      uint32_t vx = bits4_to_bytes(ub & 0xFu), vy = bits4_to_bytes((ub >> 4) & 0xFu);
-      if (any_fd) {  // warp-uniform
-        const uint32_t fb = __shfl_sync(FULL, FD, item >> 2) >> sh;
-        vx |= bits4_to_bytes(fb & 0xFu) << 1;
-        vy |= bits4_to_bytes((fb >> 4) & 0xFu) << 1;
+      for (uint32_t it = 0; it < 2; ++it) {
+        const uint32_t s = it * 16u;
+        uint32_t v0 = bits4_to_bytes((u >> s) & 0xFu), v1 = bits4_to_bytes((u >> (s + 4u)) & 0xFu);
+        uint32_t v2 = bits4_to_bytes((u >> (s + 8u)) & 0xFu), v3 = bits4_to_bytes((u >> (s + 12u)) & 0xFu);
+        if (any_fd) {  // warp-uniform
+          v0 |= bits4_to_bytes((f >> s) & 0xFu) << 1; v1 |= bits4_to_bytes((f >> (s + 4u)) & 0xFu) << 1;
+          v2 |= bits4_to_bytes((f >> (s + 8u)) & 0xFu) << 1; v3 |= bits4_to_bytes((f >> (s + 12u)) & 0xFu) << 1;
+        }
+        sts_v4(my_st + w * 32u + (hs ^ s), v0, v1, v2, v3);
       }
-      sts_v2(st0_a + item * 8u + (item >> (2u + lg)) * (st_stride - 32u * Wq), vx, vy);   // run (item >> (2 + lg)) starts at st0 + run * st_stride
     }
     // per-run walk entry: CSR / row bases, status base, longest row and row format
     const uint32_t col_a = tr_a + (h1.x & 0xFFFFu);
-    const uint32_t my_st = st0_a + g * st_stride;
     if (w == 0) sts_v4(tab_a + g * 16u, col_a, tr_a + (uint32_t)sizeof(TopoHeader), my_st, max_deg | (ell << 16));
     __syncwarp();
     // second link of the group I shall issue (its slot id, requested when I drew my ticket, has arrived by now — asking for

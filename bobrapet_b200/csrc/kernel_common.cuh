@@ -84,6 +84,12 @@ DI uint32_t spread4(uint32_t x) {  // inverse of squeeze4
   return x;
 }
 DI uint32_t bits4_to_bytes(uint32_t nib) { return (nib * 0x00204081u) & 0x01010101u; }  // 4 bits -> 4 0/1 bytes
+// byte permute with the full PTX selector: bit 3 of a selector nibble replicates the sign of the chosen byte
+DI uint32_t prmt(uint32_t a, uint32_t b, uint32_t sel) {
+  uint32_t r;
+  asm("prmt.b32 %0, %1, %2, %3;" : "=r"(r) : "r"(a), "r"(b), "r"(sel));
+  return r;
+}
 DI uint32_t get_nibble(const uint8_t* base, uint32_t i) {
   const uint32_t v = (base[i >> 1] >> ((i & 1u) * 4u)) & 0xFu;
   return v == 15u ? 0u : v;
