@@ -19,7 +19,8 @@
 // groups in flight adapts by itself (a warp waiting at a barrier IS a group in flight), and a CTA keeps 24 warps fed
 // from 33 slot groups where a private double-buffered ring per warp would allow only 16 warps.  The chain run ->
 // slot id -> slot entry of group t + NG is fetched by the R lanes that own its runs while the warp works on group t
-// (first link before the barrier wait, second after it), and those lanes issue the copies from their own registers.
+// (first link before the barrier wait, second after stage C, landing in shared memory so that it holds no registers through
+// the walk), and those lanes issue the copies.
 // A dead / oversized slot is marked by a zero header written before the arrive, a run deferred to the general kernel by
 // an all-ones header word.
 //
@@ -248,52 +249,43 @@ __global__ void __launch_bounds__(32 * PACK_MAX_WARPS, PACK_MIN_BLOCKS) frontier
   // issue 0 (lq == 0) hold the group my warp will issue when it is done with the current one.
   const uint32_t GB = 32u >> (5 - lg);        // = Wq: issues per prologue batch
   const uint32_t lq = lane >> (5 - lg), lr = lane & (R - 1u);   // my pair inside a batch: issue lq, run lr
-  uint32_t pf_sid = 0xFFFFFFFFu, pf_run = 0xFFFFFFFFu, pf_lo = 0, pf_hi = 0, pf_bytes = 0, pf_meta = 0;
+  uint32_t pf_sid = 0xFFFFFFFFu;
   auto load_sid = [&](uint32_t t, bool mine) {   // first link: my run's topology slot id (the head word of its state record)
-    pf_sid = 0xFFFFFFFFu; pf_run = 0xFFFFFFFFu;
+    pf_sid = 0xFFFFFFFFu;
     if (mine && t < T) {
       const uint32_t r = ((blockIdx.x + t * gridDim.x) << (5 - lg)) + lr;
-      if (r < N) {
-        pf_run = r;
-        pf_sid = __ldg(reinterpret_cast<const uint32_t*>(P.state + (size_t)r * P.state_stride));
-      }
+      if (r < N) pf_sid = __ldg(reinterpret_cast<const uint32_t*>(P.state + (size_t)r * P.state_stride));
     }
   };
-  auto load_ent = [&]() {                        // second link: the slot entry (address, bytes, meta)
-    pf_lo = 0; pf_hi = 0; pf_bytes = 0; pf_meta = 0;
-    if (pf_sid < P.n_slots) {
-      const uint4 v = __ldg(reinterpret_cast<const uint4*>(P.slots + pf_sid));
-      pf_lo = v.x; pf_hi = v.y; pf_bytes = v.z; pf_meta = v.w;
-    }
-  };
-  // issue the copies of group t into slot group `sg`, which thereby starts its use number `use`; `mine`: my lane owns a run of it
-  auto issue = [&](uint32_t t, uint32_t sg, uint32_t use, bool mine) {
+  // issue the copies of group t into slot group `sg`, which thereby starts its use number `use`; `mine`: my lane owns a run of
+  // it; `ent`: my run's slot entry (address, bytes, meta), all zero for a slot id out of range
+  auto issue = [&](uint32_t t, uint32_t sg, uint32_t use, bool mine, const uint4 ent) {
     if (t < T && mine) {
       const uint32_t buf = groups_a + sg * group_bytes;
       const uint32_t bar = bars + 8u * sg;
       const uint32_t tb = buf + R * P.state_stride + lr * P.topo_buf_bytes;   // my run's topology buffer
-      const bool valid = pf_run != 0xFFFFFFFFu;
-      const bool dfr = valid && P.defer_list != nullptr && (pf_meta >> 16) != 0;  // topology with parallel steps
-      const bool ok = valid && !dfr && (pf_lo | pf_hi) != 0 && pf_bytes <= P.topo_buf_bytes;
+      const uint32_t first = (blockIdx.x + t * gridDim.x) << (5 - lg);
+      const bool valid = first + lr < N;
+      const bool dfr = valid && P.defer_list != nullptr && (ent.w >> 16) != 0;  // topology with parallel steps
+      const bool ok = valid && !dfr && (ent.x | ent.y) != 0 && ent.z <= P.topo_buf_bytes;
       if (!ok) sts_v4(tb, dfr ? 0xFFFFFFFFu : 0u, 0u, 0u, 0u);   // marker header (W = 0: dead, all-ones: deferred)
       uint32_t sbytes = 0;
-      const uint32_t first = (blockIdx.x + t * gridDim.x) << (5 - lg);
       if (lr == 0) {
         sbytes = min(R, N - first) * P.state_stride;   // the group's state records are adjacent: one copy
         sts_u32(armed_a + 4u * sg, use + 1u);          // published before my arrive: the previous use is over, this one is armed
       }
-      mbar_expect_tx(bar, (ok ? pf_bytes : 0u) + sbytes);
+      mbar_expect_tx(bar, (ok ? ent.z : 0u) + sbytes);
       if (lr == 0) bulk_g2s(buf, P.state + (size_t)first * P.state_stride, sbytes, bar);
-      if (ok) bulk_g2s(tb, reinterpret_cast<const void*>((uint64_t)pf_lo | ((uint64_t)pf_hi << 32)), pf_bytes, bar);
+      if (ok) bulk_g2s(tb, reinterpret_cast<const void*>((uint64_t)ent.x | ((uint64_t)ent.y << 32)), ent.z, bar);
     }
   };
   for (uint32_t q0 = 0; q0 < n_pro; q0 += GB) {      // prologue: GB of my issues at a time (both links of all of them in flight together)
     const bool in_pro = q0 + lq < n_pro;
     load_sid(warp + (q0 + lq) * NW, in_pro);
-    load_ent();
+    const uint4 ent = pf_sid < P.n_slots ? __ldg(reinterpret_cast<const uint4*>(P.slots + pf_sid)) : make_uint4(0u, 0u, 0u, 0u);
     for (uint32_t k = 0; k < GB && q0 + k < n_pro; ++k) {
       const uint32_t t = warp + (q0 + k) * NW;       // < NG: its slot group is t itself, use 0
-      issue(t, t, 0u, lq == k);
+      issue(t, t, 0u, lq == k, ent);
     }
   }
 
@@ -306,7 +298,8 @@ __global__ void __launch_bounds__(32 * PACK_MAX_WARPS, PACK_MIN_BLOCKS) frontier
   const uint32_t ng_magic = NG > 1u ? (uint32_t)(0x100000000ull / NG) + 1u : 0u;   // t / NG = umulhi(t, ng_magic), exact for t < 2^32 / NG (NG = 1: T <= 1, t = 0)
   for (;;) {
     uint32_t t = 0;
-    if (lane == 0) t = atomicAdd(reinterpret_cast<uint32_t*>(smem_p + 32), 1u);
+    const uint32_t lane4 = pin(lane * 4u);   // outside the branch (inside it lane is known to be 0): a single-lane atomic
+    if (lane == 0) t = atoms_add_u32(smem_base + 32u + lane4, 1u);
     t = __shfl_sync(FULL, t, 0);
     if (t >= T) break;
     const uint32_t cur_use = __umulhi(t, ng_magic), cur_sg = t - cur_use * NG;   // t / NG, t % NG
@@ -395,10 +388,27 @@ __global__ void __launch_bounds__(32 * PACK_MAX_WARPS, PACK_MIN_BLOCKS) frontier
     uint32_t FAILED = TERM & ~COMPL;
     uint32_t group, sum = 0;
     // ---------------- stage I (dag.go:422-495): per-run reductions = one sub-warp redux.or ----------------
-    {
+    // A group none of whose runs has a compensation or finally step, nor takes the realtime + topology-terminated branch
+    // (host-group runs never do), needs only the main-group facts: every fact about G1 / G2 is empty, so the general code
+    // below would mark nothing there and find compensation and finally done and not failed.
+    const bool main_only = __all_sync(FULL, (G1 | G2) == 0u && !(realtime && topo_term && !host_group));
+    const uint32_t DONE = COMPL | FAILED;
+    const uint32_t mark_ff = GM & ~COMPL & ~RUNQ & ~TERM;             // markFailFastSkipped candidates (:3289-3312)
+    if (main_only) {
+      const uint32_t bits = __reduce_or_sync(gmask, ((FAILED & GM) != 0 ? 1u : 0u) | ((GM & ~DONE) != 0 ? 2u : 0u) |
+                                                        ((GM & ~DONE & ~mark_ff) != 0 ? 4u : 0u) | (mark_ff != 0 ? 8u : 0u));
+      const bool amf = bits & 1u;
+      const bool do_ff = !host_group && fail_fast && amf;
+      if (do_ff) {
+        marked = bits & 8u;
+        pset<BF_PHASE_SKIPPED>(mark_ff, p0, p1, p2, p3);
+        TERM |= mark_ff; COMPL |= mark_ff;
+      }
+      const bool main_done = n_main == 0 || !(bits & (do_ff ? 4u : 2u));
+      group = main_done ? BF_GROUP_DONE : BF_GROUP_MAIN;
+      sum = (main_done ? BF_SUM_MAIN_DONE : 0u) | (amf ? BF_SUM_MAIN_FAILED : 0u) | BF_SUM_COMP_DONE | BF_SUM_FINAL_DONE;
+    } else {
       uint32_t RUN = plut<BF_LUT_RUNNING>(p0, p1, p2, p3);
-      const uint32_t DONE = COMPL | FAILED;
-      const uint32_t mark_ff = GM & ~COMPL & ~RUNQ & ~TERM;           // markFailFastSkipped candidates (:3289-3312)
       const uint32_t mark_cs = G1 & ~COMPL & ~RUN & ~FAILED & ~TERM;   // markCompensationsSkipped candidates (:3314-3342)
       uint32_t bits = ((FAILED & GM) != 0 ? 1u : 0u) | ((GM & ~DONE) != 0 ? 2u : 0u) | ((GM & ~DONE & ~mark_ff) != 0 ? 4u : 0u) |
                       ((G1 & ~DONE) != 0 ? 8u : 0u) | ((G1 & ~DONE & ~mark_cs) != 0 ? 16u : 0u) | ((G2 & ~DONE) != 0 ? 32u : 0u) |
@@ -447,10 +457,10 @@ __global__ void __launch_bounds__(32 * PACK_MAX_WARPS, PACK_MIN_BLOCKS) frontier
       else group = BF_GROUP_DONE;
       sum = (main_done ? BF_SUM_MAIN_DONE : 0u) | (amf ? BF_SUM_MAIN_FAILED : 0u) | (comp_done ? BF_SUM_COMP_DONE : 0u) |
             (final_done ? BF_SUM_FINAL_DONE : 0u) | (acf ? BF_SUM_COMP_FAILED : 0u) | (aff ? BF_SUM_FINAL_FAILED : 0u);
-      if (host_group) {
-        group = (rflags >> BF_RF_HOST_GROUP_SHIFT) & 3u;
-        sum = 0;
-      }
+    }
+    if (host_group) {
+      group = (rflags >> BF_RF_HOST_GROUP_SHIFT) & 3u;
+      sum = 0;
     }
     uint32_t summary = sum | group;
 
@@ -494,8 +504,12 @@ __global__ void __launch_bounds__(32 * PACK_MAX_WARPS, PACK_MIN_BLOCKS) frontier
     if (w == 0) sts_v4(tab_a + g * 16u, col_a, tr_a + (uint32_t)sizeof(TopoHeader), my_st, max_deg | (ell << 16));
     __syncwarp();
     // second link of the group I shall issue (its slot id, requested when I drew my ticket, has arrived by now — asking for
-    // it right behind the barrier wait stalled every trip for a DRAM round trip); consumed by issue() at the end of the trip
-    load_ent();
+    // it right behind the barrier wait stalled every trip for a DRAM round trip); consumed by issue() at the end of the trip.
+    // The entry lands in shared memory, not in registers that would stay live through the walk: in the head of state record
+    // lr of this slot group, which nothing reads once the planes above are loaded (the __syncwarp orders those reads first)
+    // and which the re-arm overwrites only after issue() has read the entry back.
+    const uint32_t ent_a = grp_a + lr * P.state_stride;
+    if (lq == 0) cp_async16(ent_a, P.slots + (pf_sid < P.n_slots ? pf_sid : 0u), pf_sid < P.n_slots ? 16u : 0u);
     // ------------- stage D: walk the needs rows (dag.go:2711-2733) -------------
     uint32_t met_w, fd_w;
     const WalkCtx wctx{tab_a, grp_a + R * P.state_stride + (uint32_t)sizeof(TopoHeader), P.topo_buf_bytes, st0_a, st_stride};
@@ -608,7 +622,12 @@ __global__ void __launch_bounds__(32 * PACK_MAX_WARPS, PACK_MIN_BLOCKS) frontier
     lane_evals += (w == 0 && live) ? S : 0u;
 
     __syncwarp();  // every lane is done with this slot group's buffers
-    issue(t + NG, cur_sg, cur_use + 1u, lq == 0);  // re-arm it with group t + NG (consumed by whichever warp draws that ticket)
+    uint4 ent = make_uint4(0u, 0u, 0u, 0u);
+    if (lq == 0) {
+      cp_async_wait_all();
+      ent = lds_v4(ent_a);
+    }
+    issue(t + NG, cur_sg, cur_use + 1u, lq == 0, ent);  // re-arm it with group t + NG (consumed by whichever warp draws that ticket)
 #ifdef PACK_TRACE
     if (t == 0 && lane == 0 && blockIdx.x < 160) g_trace[tr_launch][blockIdx.x][1] = tr_first;
     tr_last = gtime();

@@ -40,6 +40,20 @@ DI void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
                "l"(src), "r"(bytes), "r"(bar)
                : "memory");
 }
+// 16 bytes global -> shared through the L2 (src_bytes = 0: the destination is zero-filled and nothing is read);
+// complete for the issuing thread after cp_async_wait_all
+DI void cp_async16(uint32_t dst, const void* src, uint32_t src_bytes) {
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(src_bytes) : "memory");
+}
+DI void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
+// shared-memory fetch-and-add.  An atomic on a warp-uniform address under a lane predicate, atomicAdd or inline PTX alike,
+// is compiled to a warp-aggregated atomic (lane id, vote, FLO, two POPC and a shuffle around the one ATOMS); a caller that
+// means ONE thread passes an address that depends on the lane (e.g. + lane * 4, zero for the lane that executes it).
+DI uint32_t atoms_add_u32(uint32_t a, uint32_t v) {
+  uint32_t r;
+  asm volatile("atom.shared.add.u32 %0, [%1], %2;" : "=r"(r) : "r"(a), "r"(v) : "memory");
+  return r;
+}
 DI void sts_zero16(uint32_t a) { asm volatile("st.shared.v4.u32 [%0], {%1, %1, %1, %1};" ::"r"(a), "r"(0u) : "memory"); }
 DI void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
 
